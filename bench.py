@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- loghisto hot path on B200: samples/s, HBM roofline fraction, CPU baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic float64
 samples: ingest (bucket index + increment) of the whole batch, then the
@@ -18,6 +18,9 @@ bucket->percentile reduction, result read back to the host.
 
 --impl reference times that CPU port alone (the Go reference cannot be built
 here: no Go toolchain in the image; see DESIGN.md).
+
+--dump-outputs DIR writes what the last timed step returned (counts, sums,
+avgs, pkeys, pvals of every histogram) as DIR/<name>.npy, float64.
 """
 import argparse
 import json
@@ -65,7 +68,16 @@ def parse_args():
     ap.add_argument("--debug-steps", action="store_true", help="print every timed step's kernel time to stderr")
     ap.add_argument("--nccl-defaults", action="store_true", help="do not set NCCL_MAX_NCHANNELS / NCCL_CGA_CLUSTER_SIZE")
     ap.add_argument("--reserve-sms", type=int, default=-1, help="SMs K1 leaves free for the snapshot stream (default: 0 at N=1, 2 at N>1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (the reduction of every "
+                         "histogram) as DIR/<name>.npy in float64; the inputs are a function of the arguments only, "
+                         "so two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm hands no arrays back")
+    return a
 
 
 def measured_traffic(workload, n):
@@ -394,6 +406,15 @@ def api_leg(device, kind):
 
 
 # ----------------------------------------------------------------- GPU arm
+def dump_outputs(out_dir, red):
+    """Writes the Reduced of one snapshot, every field as float64: H x (at most 32 percentiles) values, far below 64 MB,
+    so nothing is sampled.  int32 keys convert exactly, and so do the uint64 counts (below 2^53 at any bench size)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("counts", "sums", "avgs", "pkeys", "pvals"):
+        np.save(os.path.join(out_dir, name + ".npy"), getattr(red, name).astype(np.float64))
+
+
 def default_n(workload, world):
     if workload == "c5":
         return 100_000_000
@@ -736,6 +757,8 @@ def run_b200(a):
                           "reference itself cannot run" % ns,
                 "host_cpus": os.cpu_count(), "cpu_quota_cores": cpu_quota_cores(), "thread_ladder_samples_per_s": ladder,
                 "dense_private_arrays_all_cores_value": dense}
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, red)
         print(json.dumps(line))
         sys.stdout.flush()
     eng.close()
