@@ -250,6 +250,43 @@ LH_API lh_status lh_snapshot_allreduce(lh_ctx *ctx, uint32_t include_counters, u
 LH_API lh_status lh_comm_allreduce_ms(lh_ctx *ctx, uint64_t seq, float *ms);
 LH_API lh_status lh_comm_info(lh_ctx *ctx, lh_comm_stats *out);
 
+/* ---- windows: statistics over more than one interval, kept on the device ------------------------------------------
+ * One optional accumulator per context, off until lh_window_configure.  It holds the uint64 bucket sums (and counter
+ * sums) of
+ *   intervals = K (1..LH_MAX_WINDOW_INTERVALS)  the last K folded snapshots (sliding window), or
+ *   intervals = 0                               every snapshot folded since it was configured (lifetime).
+ *
+ *   lh_window_configure  (re)allocate and zero; LH_ERR_STATE while a snapshot is open.  The dense accumulator takes
+ *                        H * 512 KiB of device memory.
+ *   lh_window_release    free it; window calls then return LH_ERR_STATE until the next configure
+ *   lh_window_fold       between lh_snapshot_begin (+ lh_snapshot_allreduce, or an in-place reduction through
+ *                        lh_snapshot_device) and lh_snapshot_end, at most once per snapshot: adds what the open
+ *                        snapshot's reduction reads (the all-ranks sums after lh_snapshot_allreduce) and, when the
+ *                        window is full, subtracts the snapshot folded K folds earlier.  uint64 adds and subtracts are
+ *                        exact mod 2^64: a histogram that leaves the window comes back to all-zero cells.  One
+ *                        snapshot-stream synchronisation (the size of the sparse copy kept for the eviction).
+ *   lh_window_reduce     processHistograms over the window, with or without an open snapshot; same outputs and
+ *                        conventions as lh_snapshot_reduce (a histogram absent from every held interval is absent)
+ *   lh_window_export     the window as sparse lists; counter_deltas = counter sums over the window.  Pointers stay
+ *                        valid until the next lh_window_export / lh_window_release / lh_window_configure / lh_destroy
+ * Window calls never touch the snapshot's own results: outstanding lh_snapshot_reduce_async tickets and the buffers
+ * of lh_snapshot_export stay as they were. */
+#define LH_MAX_WINDOW_INTERVALS 1024
+typedef struct lh_window_stats {
+    uint32_t intervals;      /* configured K; 0 = lifetime */
+    uint32_t held;           /* snapshots currently inside the window (<= K) */
+    uint64_t folds;          /* lh_window_fold calls since the last configure */
+    uint64_t entries_held;   /* sparse (key,count) entries kept for eviction */
+    uint64_t device_bytes;   /* device memory the window holds */
+} lh_window_stats;
+LH_API lh_status lh_window_configure(lh_ctx *ctx, uint32_t intervals);
+LH_API lh_status lh_window_release(lh_ctx *ctx);
+LH_API lh_status lh_window_fold(lh_ctx *ctx);
+LH_API lh_status lh_window_reduce(lh_ctx *ctx, const double *percentiles, uint32_t np, uint64_t *counts,
+                                  double *sums, double *avgs, int32_t *pkeys, double *pvals);
+LH_API lh_status lh_window_export(lh_ctx *ctx, lh_sparse *out);
+LH_API lh_status lh_window_info(lh_ctx *ctx, lh_window_stats *out);
+
 /* ---- scalar helpers, evaluated ON THE DEVICE (parity probes for tests) --- */
 /* out[i] = compress(values[i]) exactly as the ingest kernels compute it
  * (mode 0: production fast path + exact fallback; mode 1: exact path only) */

@@ -62,6 +62,16 @@ class lh_sparse(C.Structure):
     ]
 
 
+class lh_window_stats(C.Structure):
+    _fields_ = [
+        ("intervals", C.c_uint32), ("held", C.c_uint32), ("folds", C.c_uint64),
+        ("entries_held", C.c_uint64), ("device_bytes", C.c_uint64),
+    ]
+
+
+LH_MAX_WINDOW_INTERVALS = 1024
+
+
 class lh_stats(C.Structure):
     _fields_ = [
         ("samples", C.c_uint64), ("counter_ops", C.c_uint64), ("dropped", C.c_uint64),
@@ -109,6 +119,12 @@ SIGNATURES = {
     "lh_snapshot_allreduce": (_i32, [_vp, _u32, C.POINTER(_u64)]),
     "lh_comm_allreduce_ms": (_i32, [_vp, _u64, C.POINTER(C.c_float)]),
     "lh_comm_info": (_i32, [_vp, C.POINTER(lh_comm_stats)]),
+    "lh_window_configure": (_i32, [_vp, _u32]),
+    "lh_window_release": (_i32, [_vp]),
+    "lh_window_fold": (_i32, [_vp]),
+    "lh_window_reduce": (_i32, [_vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
+    "lh_window_export": (_i32, [_vp, C.POINTER(lh_sparse)]),
+    "lh_window_info": (_i32, [_vp, C.POINTER(lh_window_stats)]),
     "lh_keyed_kernel_name": (C.c_char_p, [_vp]),
     "lh_compress_f64": (_i32, [_vp, _vp, _sz, _vp, C.c_int, _vp]),
     "lh_decompress_table": (_i32, [_vp, _vp]),

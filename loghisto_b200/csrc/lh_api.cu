@@ -135,6 +135,46 @@ struct PeerMap {                                   // one remote rank as mapped 
     bool ipc = false;                              // pointers came from cudaIpcOpenMemHandle (must be closed)
 };
 
+// Sparse lists of one view (k_reduce's non-empty counts -> k_scan_nnz -> k_export) and their pinned host mirrors.
+// The snapshot and the window each own one set, so neither disturbs what the other handed out.
+struct ExportBufs {
+    uint32_t *d_nnz = nullptr, *d_offsets = nullptr;   // [H], [H+1]
+    uint32_t *h_offsets = nullptr;
+    unsigned long long *h_counters = nullptr;          // [C]
+    short *d_keys = nullptr, *h_keys = nullptr;
+    unsigned long long *d_counts = nullptr, *h_counts = nullptr;
+    size_t cap = 0;                                    // entries the key / count buffers hold
+};
+
+// One folded snapshot as the window keeps it until it leaves the window (device memory only).
+struct WinSlot {
+    uint32_t *d_offsets = nullptr;            // [H+1]
+    uint32_t *d_flags = nullptr;              // [H]
+    unsigned long long *d_counters = nullptr; // [C]
+    short *d_keys = nullptr;
+    unsigned long long *d_counts = nullptr;
+    size_t cap = 0;
+    uint64_t entries = 0;
+};
+
+struct Window {
+    uint32_t intervals = 0;                   // K; 0 = lifetime
+    uint64_t folds = 0;
+    uint64_t folded_snapshot = 0;             // lh_stats.snapshots of the snapshot folded last (one fold per snapshot)
+    unsigned long long *d_acc = nullptr;      // [H][65536]
+    uint32_t *d_flags = nullptr;              // [H] 0 / 1 / 3, as a snapshot's
+    uint32_t *d_levels = nullptr;             // [2][H] held intervals that touched h at level >= 1, at level 3
+    unsigned long long *d_counters = nullptr; // [C]
+    // sliding: K + 1 slots, so the capture of fold f never lands on fold f - K before k_window_apply has subtracted
+    // it; lifetime: one slot, overwritten by every fold
+    std::vector<WinSlot> ring;
+    uint32_t *h_total = nullptr;              // pinned: entries of the slot being captured
+    double *d_ps = nullptr;
+    char *d_res = nullptr, *h_res = nullptr;  // one result slot, laid out as the snapshot's
+    bool nnz_valid = false;                   // x.d_nnz holds the accumulator's non-empty counts
+    ExportBufs x;
+};
+
 }  // namespace
 
 struct lh_ctx {
@@ -160,12 +200,8 @@ struct lh_ctx {
     uint32_t res_np[3] = {0, 0, 0};
     uint64_t res_ticket[2] = {0, 0};
     uint64_t next_ticket = 1;
-    uint32_t *d_nnz = nullptr, *d_offsets = nullptr;
-    short *d_x_keys = nullptr; unsigned long long *d_x_counts = nullptr; size_t x_cap = 0;
-    // pinned host mirrors
-    uint32_t *h_offsets = nullptr;
-    short *h_x_keys = nullptr; unsigned long long *h_x_counts = nullptr; size_t hx_cap = 0;
-    unsigned long long *h_counter_deltas = nullptr;
+    ExportBufs x;                       // lh_snapshot_export's lists (d_nnz also takes every snapshot reduction's counts)
+    Window *win = nullptr;              // lh_window_*; null until lh_window_configure
     // staging ring
     std::vector<Slot> slots;
     uint64_t slot_seq = 0;
@@ -694,6 +730,42 @@ bool is_pinned_or_managed(const void *p) {
     return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
 }
 
+cudaError_t export_bufs_alloc(ExportBufs &x, size_t H, size_t C) {
+    cudaError_t e = cudaMalloc(&x.d_nnz, H * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&x.d_offsets, (H + 1) * 4);
+    if (e == cudaSuccess) e = cudaMallocHost(&x.h_offsets, (H + 1) * 4);
+    if (e == cudaSuccess) e = cudaMallocHost(&x.h_counters, C * 8);
+    return e;
+}
+
+void export_bufs_free_lists(ExportBufs &x) {
+    cudaFree(x.d_keys); cudaFree(x.d_counts);
+    if (x.h_keys) cudaFreeHost(x.h_keys);
+    if (x.h_counts) cudaFreeHost(x.h_counts);
+    x.d_keys = nullptr; x.d_counts = nullptr; x.h_keys = nullptr; x.h_counts = nullptr; x.cap = 0;
+}
+
+void export_bufs_free(ExportBufs &x) {
+    export_bufs_free_lists(x);
+    cudaFree(x.d_nnz); cudaFree(x.d_offsets);
+    if (x.h_offsets) cudaFreeHost(x.h_offsets);
+    if (x.h_counters) cudaFreeHost(x.h_counters);
+    x = ExportBufs{};
+}
+
+void window_free(Window *w) {
+    if (!w) return;
+    cudaFree(w->d_acc); cudaFree(w->d_flags); cudaFree(w->d_levels); cudaFree(w->d_counters);
+    for (auto &sl : w->ring) {
+        cudaFree(sl.d_offsets); cudaFree(sl.d_flags); cudaFree(sl.d_counters); cudaFree(sl.d_keys); cudaFree(sl.d_counts);
+    }
+    if (w->h_total) cudaFreeHost(w->h_total);
+    cudaFree(w->d_ps); cudaFree(w->d_res);
+    if (w->h_res) cudaFreeHost(w->h_res);
+    export_bufs_free(w->x);
+    delete w;
+}
+
 }  // namespace
 
 // =========================================================== lifecycle
@@ -808,10 +880,7 @@ extern "C" lh_status lh_create(const lh_config *cfg, lh_ctx **out) {
         LH_CREATE_CUDA(cudaMallocHost(&ctx->h_res[i], res_bytes));
         LH_CREATE_CUDA(cudaEventCreateWithFlags(&ctx->res_done[i], cudaEventDisableTiming));
     }
-    LH_CREATE_CUDA(cudaMalloc(&ctx->d_nnz, (size_t)ctx->H * 4));
-    LH_CREATE_CUDA(cudaMalloc(&ctx->d_offsets, ((size_t)ctx->H + 1) * 4));
-    LH_CREATE_CUDA(cudaMallocHost(&ctx->h_offsets, ((size_t)ctx->H + 1) * 4));
-    LH_CREATE_CUDA(cudaMallocHost(&ctx->h_counter_deltas, counter_bytes));
+    LH_CREATE_CUDA(export_bufs_alloc(ctx->x, ctx->H, ctx->C));
 
     ctx->slots.resize(nslots);   // pinned + device memory of a slot is allocated the first time it is handed out
     for (auto &sl : ctx->slots) {
@@ -878,12 +947,9 @@ extern "C" lh_status lh_destroy(lh_ctx *ctx) {
         if (ctx->h_res[i]) cudaFreeHost(ctx->h_res[i]);
         if (ctx->res_done[i]) cudaEventDestroy(ctx->res_done[i]);
     }
-    cudaFree(ctx->d_nnz); cudaFree(ctx->d_offsets);
-    cudaFree(ctx->d_x_keys); cudaFree(ctx->d_x_counts);
-    if (ctx->h_offsets) cudaFreeHost(ctx->h_offsets);
-    if (ctx->h_x_keys) cudaFreeHost(ctx->h_x_keys);
-    if (ctx->h_x_counts) cudaFreeHost(ctx->h_x_counts);
-    if (ctx->h_counter_deltas) cudaFreeHost(ctx->h_counter_deltas);
+    export_bufs_free(ctx->x);
+    window_free(ctx->win);
+    ctx->win = nullptr;
     for (auto &sl : ctx->slots) {
         if (sl.h) cudaFreeHost(sl.h);
         cudaFree(sl.d);
@@ -1202,25 +1268,82 @@ View snapshot_view(lh_ctx *ctx) {
     return v;
 }
 
+// enqueue the percentiles' H2D and K3 over (buckets, flags) into the packed result array d, on the snapshot stream
+lh_status launch_reduce(lh_ctx *ctx, const unsigned long long *buckets, const uint32_t *flags, const double *ps, uint32_t np,
+                        double *d_ps, char *d, uint32_t *d_nnz) {
+    cudaStream_t s = ctx->snap_stream;
+    const ResLayout l = res_layout(ctx->H, np);
+    if (np) {
+        LH_CUDA(ctx, cudaMemcpyAsync(d_ps, ps, np * sizeof(double), cudaMemcpyHostToDevice, s));
+    }
+    // shared-memory window path when the 2*win-1 cells fit comfortably (two CTAs per SM); the dense path otherwise
+    const size_t cells = (size_t)2 * ctx->pc.win - 1;
+    const uint32_t smem_cells = cells * 8 <= (size_t)100 * 1024 ? (uint32_t)cells : 0u;
+    k_reduce<<<ctx->H, K3_THREADS, (size_t)smem_cells * 8, s>>>(buckets, flags, ctx->pc.win, ctx->d_decomp, d_ps, (int)np,
+                                           (unsigned long long *)(d + l.count), (double *)(d + l.sum), (double *)(d + l.avg),
+                                           (int *)(d + l.pkeys), (double *)(d + l.pvals), d_nnz, smem_cells);
+    LH_CUDA(ctx, cudaGetLastError());
+    ctx->stats.kernel_launches++;
+    return LH_OK;
+}
+
+// copy the packed results of h (laid out by res_layout(H, np)) into the caller's arrays (any may be NULL)
+void unpack_results(const char *h, size_t H, uint32_t np, uint64_t *counts, double *sums, double *avgs, int32_t *pkeys,
+                    double *pvals) {
+    const ResLayout l = res_layout(H, np);
+    if (counts) memcpy(counts, h + l.count, H * 8);
+    if (sums) memcpy(sums, h + l.sum, H * 8);
+    if (avgs) memcpy(avgs, h + l.avg, H * 8);
+    if (pvals && np) memcpy(pvals, h + l.pvals, H * np * 8);
+    if (pkeys && np) memcpy(pkeys, h + l.pkeys, H * np * 4);
+}
+
+// Sparse lists of (buckets, flags) into x, whose d_nnz already holds K3's non-empty counts of that view, plus a copy
+// of `counters`.  Synchronises the snapshot stream (twice when there is anything to list).
+lh_status export_lists(lh_ctx *ctx, ExportBufs &x, const unsigned long long *buckets, const uint32_t *flags,
+                       const unsigned long long *counters, lh_sparse *out) {
+    cudaStream_t s = ctx->snap_stream;
+    k_scan_nnz<<<1, 1024, 0, s>>>(x.d_nnz, ctx->H, x.d_offsets);
+    LH_CUDA(ctx, cudaGetLastError());
+    LH_CUDA(ctx, cudaMemcpyAsync(x.h_offsets, x.d_offsets, ((size_t)ctx->H + 1) * 4, cudaMemcpyDeviceToHost, s));
+    LH_CUDA(ctx, cudaMemcpyAsync(x.h_counters, counters, (size_t)ctx->C * 8, cudaMemcpyDeviceToHost, s));
+    LH_CUDA(ctx, cudaStreamSynchronize(s));
+    const size_t total = x.h_offsets[ctx->H];
+    if (total > x.cap) {
+        size_t cap = std::max<size_t>(total, 4096) * 2;
+        export_bufs_free_lists(x);
+        LH_CUDA(ctx, cudaMalloc(&x.d_keys, cap * 2));
+        LH_CUDA(ctx, cudaMalloc(&x.d_counts, cap * 8));
+        LH_CUDA(ctx, cudaMallocHost(&x.h_keys, cap * 2));
+        LH_CUDA(ctx, cudaMallocHost(&x.h_counts, cap * 8));
+        x.cap = cap;
+    }
+    if (total) {
+        k_export<<<ctx->H, K3_THREADS, 0, s>>>(buckets, flags, ctx->pc.win, x.d_offsets, x.d_keys, x.d_counts);
+        LH_CUDA(ctx, cudaGetLastError());
+        ctx->stats.kernel_launches += 2;
+        LH_CUDA(ctx, cudaMemcpyAsync(x.h_keys, x.d_keys, total * 2, cudaMemcpyDeviceToHost, s));
+        LH_CUDA(ctx, cudaMemcpyAsync(x.h_counts, x.d_counts, total * 8, cudaMemcpyDeviceToHost, s));
+        LH_CUDA(ctx, cudaStreamSynchronize(s));
+    }
+    ctx->stats.d2h_bytes += total * 10 + ((size_t)ctx->H + 1) * 4 + (size_t)ctx->C * 8;
+    out->offsets = x.h_offsets;
+    out->keys = x.h_keys;
+    out->counts = reinterpret_cast<const uint64_t *>(x.h_counts);
+    out->counter_deltas = reinterpret_cast<const uint64_t *>(x.h_counters);
+    out->total_entries = total;
+    return LH_OK;
+}
+
 // enqueue K3 + one packed D2H for the open snapshot into result slot `slot`
 lh_status enqueue_reduce(lh_ctx *ctx, const double *ps, uint32_t np, int slot) {
     cudaStream_t s = ctx->snap_stream;
     const ResLayout l = res_layout(ctx->H, np);
     const View v = snapshot_view(ctx);
-    if (np) {
-        LH_CUDA(ctx, cudaMemcpyAsync(ctx->d_ps[slot], ps, np * sizeof(double), cudaMemcpyHostToDevice, s));
-    }
     char *d = ctx->d_res[slot];
-    // shared-memory window path when the 2*win-1 cells fit comfortably (two CTAs per SM); the dense path otherwise
-    const size_t cells = (size_t)2 * ctx->pc.win - 1;
-    const uint32_t smem_cells = cells * 8 <= (size_t)100 * 1024 ? (uint32_t)cells : 0u;
-    k_reduce<<<ctx->H, K3_THREADS, (size_t)smem_cells * 8, s>>>(v.buckets, v.flags, ctx->pc.win, ctx->d_decomp, ctx->d_ps[slot], (int)np,
-                                           (unsigned long long *)(d + l.count), (double *)(d + l.sum), (double *)(d + l.avg),
-                                           (int *)(d + l.pkeys), (double *)(d + l.pvals), ctx->d_nnz, smem_cells);
-    LH_CUDA(ctx, cudaGetLastError());
+    if (lh_status st = launch_reduce(ctx, v.buckets, v.flags, ps, np, ctx->d_ps[slot], d, ctx->x.d_nnz)) return st;
     LH_CUDA(ctx, cudaMemcpyAsync(ctx->h_res[slot], d, l.total, cudaMemcpyDeviceToHost, s));
     LH_CUDA(ctx, cudaEventRecord(ctx->res_done[slot], s));
-    ctx->stats.kernel_launches++;
     ctx->stats.d2h_bytes += l.total;
     ctx->nnz_valid = true;
     ctx->res_np[slot] = np;
@@ -1267,15 +1390,7 @@ extern "C" lh_status lh_snapshot_result(lh_ctx *ctx, uint64_t ticket, uint64_t *
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (e != cudaSuccess) return fail(ctx, LH_ERR_CUDA, "cudaEventSynchronize(result)", e);
     if (ctx->res_ticket[slot] != ticket) return fail(ctx, LH_ERR_STATE, "ticket expired while waiting");
-    const size_t H = ctx->H;
-    const uint32_t np = ctx->res_np[slot];
-    const ResLayout l = res_layout(H, np);
-    const char *h = ctx->h_res[slot];
-    if (counts) memcpy(counts, h + l.count, H * 8);
-    if (sums) memcpy(sums, h + l.sum, H * 8);
-    if (avgs) memcpy(avgs, h + l.avg, H * 8);
-    if (pvals && np) memcpy(pvals, h + l.pvals, H * np * 8);
-    if (pkeys && np) memcpy(pkeys, h + l.pkeys, H * np * 4);
+    unpack_results(ctx->h_res[slot], ctx->H, ctx->res_np[slot], counts, sums, avgs, pkeys, pvals);
     return LH_OK;
 }
 
@@ -1291,7 +1406,6 @@ extern "C" lh_status lh_snapshot_export(lh_ctx *ctx, lh_sparse *out) {
     LH_ENTER(ctx);
     if (!out) return fail(ctx, LH_ERR_INVALID, "out is NULL");
     if (!ctx->frozen) return fail(ctx, LH_ERR_STATE, "no snapshot in progress");
-    cudaStream_t s = ctx->snap_stream;
     const View v = snapshot_view(ctx);
     if (!ctx->nnz_valid) {
         // non-empty bucket counts come out of K3: run it with no percentiles into the scratch result slot, which never
@@ -1299,39 +1413,7 @@ extern "C" lh_status lh_snapshot_export(lh_ctx *ctx, lh_sparse *out) {
         lh_status st = enqueue_reduce(ctx, nullptr, 0, 2);
         if (st != LH_OK) return st;
     }
-    k_scan_nnz<<<1, 1024, 0, s>>>(ctx->d_nnz, ctx->H, ctx->d_offsets);
-    LH_CUDA(ctx, cudaGetLastError());
-    LH_CUDA(ctx, cudaMemcpyAsync(ctx->h_offsets, ctx->d_offsets, ((size_t)ctx->H + 1) * 4, cudaMemcpyDeviceToHost, s));
-    LH_CUDA(ctx, cudaMemcpyAsync(ctx->h_counter_deltas, v.counters, (size_t)ctx->C * 8, cudaMemcpyDeviceToHost, s));
-    LH_CUDA(ctx, cudaStreamSynchronize(s));
-    const size_t total = ctx->h_offsets[ctx->H];
-    if (total > ctx->x_cap) {
-        size_t cap = std::max<size_t>(total, 4096) * 2;
-        cudaFree(ctx->d_x_keys); cudaFree(ctx->d_x_counts);
-        if (ctx->h_x_keys) cudaFreeHost(ctx->h_x_keys);
-        if (ctx->h_x_counts) cudaFreeHost(ctx->h_x_counts);
-        ctx->d_x_keys = nullptr; ctx->d_x_counts = nullptr; ctx->h_x_keys = nullptr; ctx->h_x_counts = nullptr; ctx->x_cap = 0;
-        LH_CUDA(ctx, cudaMalloc(&ctx->d_x_keys, cap * 2));
-        LH_CUDA(ctx, cudaMalloc(&ctx->d_x_counts, cap * 8));
-        LH_CUDA(ctx, cudaMallocHost(&ctx->h_x_keys, cap * 2));
-        LH_CUDA(ctx, cudaMallocHost(&ctx->h_x_counts, cap * 8));
-        ctx->x_cap = cap;
-    }
-    if (total) {
-        k_export<<<ctx->H, K3_THREADS, 0, s>>>(v.buckets, v.flags, ctx->pc.win, ctx->d_offsets, ctx->d_x_keys, ctx->d_x_counts);
-        LH_CUDA(ctx, cudaGetLastError());
-        ctx->stats.kernel_launches += 2;
-        LH_CUDA(ctx, cudaMemcpyAsync(ctx->h_x_keys, ctx->d_x_keys, total * 2, cudaMemcpyDeviceToHost, s));
-        LH_CUDA(ctx, cudaMemcpyAsync(ctx->h_x_counts, ctx->d_x_counts, total * 8, cudaMemcpyDeviceToHost, s));
-        LH_CUDA(ctx, cudaStreamSynchronize(s));
-    }
-    ctx->stats.d2h_bytes += total * 10 + ((size_t)ctx->H + 1) * 4 + (size_t)ctx->C * 8;
-    out->offsets = ctx->h_offsets;
-    out->keys = ctx->h_x_keys;
-    out->counts = reinterpret_cast<const uint64_t *>(ctx->h_x_counts);
-    out->counter_deltas = reinterpret_cast<const uint64_t *>(ctx->h_counter_deltas);
-    out->total_entries = total;
-    return LH_OK;
+    return export_lists(ctx, ctx->x, v.buckets, v.flags, v.counters, out);
 }
 
 extern "C" lh_status lh_snapshot_copy_histogram(lh_ctx *ctx, uint32_t hid, uint64_t *h_out) {
@@ -1537,6 +1619,167 @@ extern "C" lh_status lh_comm_info(lh_ctx *ctx, lh_comm_stats *out) {
         // one-shot: every cell from every peer; two-shot: this rank's 1/world of the cells from every peer (and as much pushed back)
         out->last_bytes_from_peers = ctx->comm_two_shot ? cells * 8u * (ctx->comm_world - 1) / ctx->comm_world : cells * 8u * (ctx->comm_world - 1);
     }
+    return LH_OK;
+}
+
+// =========================================================== windows
+namespace {
+// offsets / flags / counters of a ring slot, on its first use
+lh_status win_slot_alloc(lh_ctx *ctx, WinSlot &sl) {
+    if (sl.d_offsets) return LH_OK;
+    LH_CUDA(ctx, cudaMalloc(&sl.d_offsets, ((size_t)ctx->H + 1) * 4));
+    LH_CUDA(ctx, cudaMalloc(&sl.d_flags, (size_t)ctx->H * 4));
+    LH_CUDA(ctx, cudaMalloc(&sl.d_counters, (size_t)ctx->C * 8));
+    return LH_OK;
+}
+
+WinSlotView win_slot_view(const WinSlot *sl) {
+    if (!sl) return WinSlotView{nullptr, nullptr, nullptr, nullptr, nullptr};
+    return WinSlotView{sl->d_offsets, sl->d_keys, sl->d_counts, sl->d_flags, sl->d_counters};
+}
+
+#define LH_WINDOW(ctx)                                                                          \
+    if (!(ctx)->win) return fail((ctx), LH_ERR_STATE, "no window configured (lh_window_configure)")
+}  // namespace
+
+extern "C" lh_status lh_window_configure(lh_ctx *ctx, uint32_t intervals) {
+    LH_ENTER(ctx);
+    if (intervals > LH_MAX_WINDOW_INTERVALS) return fail(ctx, LH_ERR_INVALID, "intervals > LH_MAX_WINDOW_INTERVALS");
+    if (ctx->frozen) return fail(ctx, LH_ERR_STATE, "lh_window_configure while a snapshot is open");
+    LH_CUDA(ctx, cudaStreamSynchronize(ctx->snap_stream));   // nothing in flight may still use the old window
+    window_free(ctx->win);
+    ctx->win = nullptr;
+    Window *w = new (std::nothrow) Window();
+    if (!w) return fail(ctx, LH_ERR_NOMEM, "window");
+    ctx->win = w;
+    w->intervals = intervals;
+    w->ring.resize(intervals ? (size_t)intervals + 1 : 1);
+    const size_t H = ctx->H, C = ctx->C, acc_bytes = H * 65536u * 8u;
+    cudaError_t e = cudaMalloc(&w->d_acc, acc_bytes);
+    if (e == cudaSuccess) e = cudaMalloc(&w->d_flags, H * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&w->d_levels, H * 8);
+    if (e == cudaSuccess) e = cudaMalloc(&w->d_counters, C * 8);
+    if (e == cudaSuccess) e = cudaMallocHost(&w->h_total, 4);
+    if (e == cudaSuccess) e = cudaMalloc(&w->d_ps, LH_MAX_PERCENTILES * sizeof(double));
+    if (e == cudaSuccess) e = cudaMalloc(&w->d_res, H * (24 + LH_MAX_PERCENTILES * 12));
+    if (e == cudaSuccess) e = cudaMallocHost(&w->h_res, H * (24 + LH_MAX_PERCENTILES * 12));
+    if (e == cudaSuccess) e = export_bufs_alloc(w->x, H, C);
+    if (e == cudaSuccess) e = cudaMemsetAsync(w->d_acc, 0, acc_bytes, ctx->snap_stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(w->d_flags, 0, H * 4, ctx->snap_stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(w->d_levels, 0, H * 8, ctx->snap_stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(w->d_counters, 0, C * 8, ctx->snap_stream);
+    if (e != cudaSuccess) {
+        window_free(w);
+        ctx->win = nullptr;
+        return fail(ctx, e == cudaErrorMemoryAllocation ? LH_ERR_NOMEM : LH_ERR_CUDA, "allocating the window", e);
+    }
+    return LH_OK;
+}
+
+extern "C" lh_status lh_window_release(lh_ctx *ctx) {
+    LH_ENTER(ctx);
+    LH_WINDOW(ctx);
+    LH_CUDA(ctx, cudaStreamSynchronize(ctx->snap_stream));
+    window_free(ctx->win);
+    ctx->win = nullptr;
+    return LH_OK;
+}
+
+// Capture the open snapshot's view as sparse lists into the next ring slot (K3's non-empty counts, the one host
+// synchronisation that sizes the slot, k_export), then fold it in and the slot of K folds ago out (k_window_apply).
+extern "C" lh_status lh_window_fold(lh_ctx *ctx) {
+    LH_ENTER(ctx);
+    LH_WINDOW(ctx);
+    Window *w = ctx->win;
+    if (!ctx->frozen) return fail(ctx, LH_ERR_STATE, "lh_window_fold without an open snapshot");
+    if (w->folded_snapshot == ctx->stats.snapshots) return fail(ctx, LH_ERR_STATE, "this snapshot has already been folded");
+    cudaStream_t s = ctx->snap_stream;
+    const View v = snapshot_view(ctx);
+    const uint32_t K = w->intervals;
+    const size_t nslots = w->ring.size();
+    WinSlot &add = w->ring[w->folds % nslots];
+    const WinSlot *sub = (K && w->folds >= K) ? &w->ring[(w->folds - K) % nslots] : nullptr;
+    if (lh_status st = win_slot_alloc(ctx, add)) return st;
+    if (!ctx->nnz_valid) {   // the snapshot's non-empty counts, exactly as lh_snapshot_export obtains them
+        if (lh_status st = enqueue_reduce(ctx, nullptr, 0, 2)) return st;
+    }
+    k_scan_nnz<<<1, 1024, 0, s>>>(ctx->x.d_nnz, ctx->H, add.d_offsets);
+    LH_CUDA(ctx, cudaGetLastError());
+    LH_CUDA(ctx, cudaMemcpyAsync(w->h_total, add.d_offsets + ctx->H, 4, cudaMemcpyDeviceToHost, s));
+    LH_CUDA(ctx, cudaMemcpyAsync(add.d_flags, v.flags, (size_t)ctx->H * 4, cudaMemcpyDeviceToDevice, s));
+    LH_CUDA(ctx, cudaMemcpyAsync(add.d_counters, v.counters, (size_t)ctx->C * 8, cudaMemcpyDeviceToDevice, s));
+    LH_CUDA(ctx, cudaStreamSynchronize(s));
+    const size_t total = *w->h_total;
+    if (total > add.cap) {   // geometric growth, as the export buffers
+        const size_t cap = std::max<size_t>(total, 4096) * 2;
+        cudaFree(add.d_keys); cudaFree(add.d_counts);
+        add.d_keys = nullptr; add.d_counts = nullptr; add.cap = 0;
+        LH_CUDA(ctx, cudaMalloc(&add.d_keys, cap * 2));
+        LH_CUDA(ctx, cudaMalloc(&add.d_counts, cap * 8));
+        add.cap = cap;
+    }
+    if (total) {
+        k_export<<<ctx->H, K3_THREADS, 0, s>>>(v.buckets, v.flags, ctx->pc.win, add.d_offsets, add.d_keys, add.d_counts);
+        LH_CUDA(ctx, cudaGetLastError());
+        ctx->stats.kernel_launches++;
+    }
+    k_window_apply<<<ctx->H, KW_THREADS, 0, s>>>(w->d_acc, w->d_flags, w->d_levels, w->d_counters, ctx->H, ctx->C,
+                                                 win_slot_view(&add), win_slot_view(sub));
+    LH_CUDA(ctx, cudaGetLastError());
+    ctx->stats.kernel_launches += 2;
+    add.entries = total;
+    w->folds++;
+    w->folded_snapshot = ctx->stats.snapshots;
+    w->nnz_valid = false;
+    return LH_OK;
+}
+
+extern "C" lh_status lh_window_reduce(lh_ctx *ctx, const double *percentiles, uint32_t np, uint64_t *counts, double *sums,
+                                      double *avgs, int32_t *pkeys, double *pvals) {
+    LH_ENTER(ctx);
+    LH_WINDOW(ctx);
+    if (np > LH_MAX_PERCENTILES || (np && !percentiles)) return fail(ctx, LH_ERR_INVALID, "bad percentile array");
+    Window *w = ctx->win;
+    const ResLayout l = res_layout(ctx->H, np);
+    if (lh_status st = launch_reduce(ctx, w->d_acc, w->d_flags, percentiles, np, w->d_ps, w->d_res, w->x.d_nnz)) return st;
+    LH_CUDA(ctx, cudaMemcpyAsync(w->h_res, w->d_res, l.total, cudaMemcpyDeviceToHost, ctx->snap_stream));
+    LH_CUDA(ctx, cudaStreamSynchronize(ctx->snap_stream));
+    ctx->stats.d2h_bytes += l.total;
+    w->nnz_valid = true;
+    unpack_results(w->h_res, ctx->H, np, counts, sums, avgs, pkeys, pvals);
+    return LH_OK;
+}
+
+extern "C" lh_status lh_window_export(lh_ctx *ctx, lh_sparse *out) {
+    LH_ENTER(ctx);
+    LH_WINDOW(ctx);
+    if (!out) return fail(ctx, LH_ERR_INVALID, "out is NULL");
+    Window *w = ctx->win;
+    if (!w->nnz_valid) {
+        if (lh_status st = launch_reduce(ctx, w->d_acc, w->d_flags, nullptr, 0, w->d_ps, w->d_res, w->x.d_nnz)) return st;
+        w->nnz_valid = true;
+    }
+    return export_lists(ctx, w->x, w->d_acc, w->d_flags, w->d_counters, out);
+}
+
+extern "C" lh_status lh_window_info(lh_ctx *ctx, lh_window_stats *out) {
+    LH_ENTER(ctx);
+    LH_WINDOW(ctx);
+    if (!out) return fail(ctx, LH_ERR_INVALID, "out is NULL");
+    const Window *w = ctx->win;
+    const size_t H = ctx->H, C = ctx->C;
+    memset(out, 0, sizeof *out);
+    out->intervals = w->intervals;
+    out->folds = w->folds;
+    const uint64_t held = w->intervals ? std::min<uint64_t>(w->folds, w->intervals) : w->folds;
+    out->held = (uint32_t)std::min<uint64_t>(held, UINT32_MAX);
+    if (w->intervals)
+        for (uint64_t i = 0; i < held; i++) out->entries_held += w->ring[(w->folds - 1 - i) % w->ring.size()].entries;
+    uint64_t bytes = H * 65536u * 8u + H * 4 + H * 8 + C * 8 + LH_MAX_PERCENTILES * 8 + H * (24 + LH_MAX_PERCENTILES * 12)
+                   + H * 4 + (H + 1) * 4 + w->x.cap * 10;
+    for (const auto &sl : w->ring)
+        if (sl.d_offsets) bytes += (H + 1) * 4 + H * 4 + C * 8 + sl.cap * 10;
+    out->device_bytes = bytes;
     return LH_OK;
 }
 

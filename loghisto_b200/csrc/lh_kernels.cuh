@@ -1417,6 +1417,46 @@ k_clear_touched(unsigned long long *__restrict__ buckets, uint32_t *__restrict__
     if (threadIdx.x == 0) flags[h] = 0;
 }
 
+// ------------------------------------------------------------------- window
+// One folded snapshot as the window keeps it: the k_export lists of its view plus its flags and counter deltas.
+struct WinSlotView {
+    const uint32_t *offsets;            // [H+1]
+    const short *keys;
+    const unsigned long long *counts;
+    const uint32_t *flags;              // [H]
+    const unsigned long long *counters; // [C]
+};
+
+// acc += the new slot, acc -= the evicted one (sub.offsets == nullptr: nothing leaves the window).  One CTA per
+// histogram; a (histogram, key) pair occurs at most once in a slot, so each pass writes distinct cells and needs no
+// atomics, and the barrier between the passes orders the add and the subtract of a key present in both.  levels[h] /
+// levels[H+h] count the held intervals that touched h at flag level >= 1 / == 3, so the window's flag is exact when
+// an interval drops out.  Counter sums ride along on a grid-stride loop.
+constexpr int KW_THREADS = 512;
+__global__ void __launch_bounds__(KW_THREADS)
+k_window_apply(unsigned long long *__restrict__ acc, uint32_t *__restrict__ acc_flags, uint32_t *__restrict__ levels,
+               unsigned long long *__restrict__ acc_counters, uint32_t H, uint32_t C, WinSlotView add, WinSlotView sub) {
+    const uint32_t h = blockIdx.x, t = threadIdx.x;
+    for (uint32_t i = h * KW_THREADS + t; i < C; i += gridDim.x * KW_THREADS)
+        acc_counters[i] += add.counters[i] - (sub.offsets ? sub.counters[i] : 0ull);
+    const uint32_t fa = add.flags[h], fs = sub.offsets ? sub.flags[h] : 0u;
+    if (!fa && !fs) return;
+    unsigned long long *hb = acc + (size_t)h * 65536u;
+    for (uint32_t i = add.offsets[h] + t; i < add.offsets[h + 1]; i += KW_THREADS)
+        hb[(unsigned short)add.keys[i]] += add.counts[i];
+    __syncthreads();
+    if (fs)
+        for (uint32_t i = sub.offsets[h] + t; i < sub.offsets[h + 1]; i += KW_THREADS)
+            hb[(unsigned short)sub.keys[i]] -= sub.counts[i];
+    if (t == 0) {
+        const uint32_t n1 = levels[h] + (fa != 0u) - (fs != 0u);
+        const uint32_t n3 = levels[H + h] + ((fa & 2u) != 0u) - ((fs & 2u) != 0u);
+        levels[h] = n1;
+        levels[H + h] = n3;
+        acc_flags[h] = n3 ? 3u : (n1 ? 1u : 0u);
+    }
+}
+
 // ---------------------------------------------------------------------- K5
 // Multi-GPU snapshot: one small kernel per rank sums, for every histogram some rank touched, the window cells of
 // ALL ranks' frozen arrays (peer-mapped device memory: direct NVLink loads, no staging copy, no library

@@ -133,24 +133,28 @@ class ShardedEngine:
             e1.record(ext)
         return ("nccl", (e0, e1))
 
-    def snapshot(self, percentiles, export: bool = False, counters: bool = False):
+    def snapshot(self, percentiles, export: bool = False, counters: bool = False, window: bool = False):
+        """window=True also folds the (all-reduced) snapshot into the engine's window (Engine.window_configure)."""
         eng = self.engine
         eng.snapshot_begin()
         try:
             if self.world > 1:
                 self._allreduce_frozen(counters)
+            if window:
+                eng.window_fold()
             red = eng.snapshot_reduce(percentiles)
             sp = eng.snapshot_export() if export else None
         finally:
             eng.snapshot_end()
         return red, sp
 
-    def snapshot_async(self, percentiles, counters: bool = False, after_swap=None):
+    def snapshot_async(self, percentiles, counters: bool = False, after_swap=None, window: bool = False):
         """begin + all-reduce + reduce + end, all enqueued; returns a handle for result() / allreduce_ms().
 
         `after_swap` (optional callable) runs right after the buffer swap and before the collective is issued:
         pipelined callers launch the next interval's ingest there, so that it is already queued on the device
-        should the collective's host call take time."""
+        should the collective's host call take time.  window=True folds the snapshot into the engine's window
+        after the collective (one snapshot-stream synchronisation)."""
         eng = self.engine
         eng.snapshot_begin()
         ar = None
@@ -159,6 +163,8 @@ class ShardedEngine:
                 after_swap()
             if self.world > 1:
                 ar = self._allreduce_frozen(counters)
+            if window:
+                eng.window_fold()
             h = eng.snapshot_reduce_async(percentiles)
         finally:
             eng.snapshot_end()

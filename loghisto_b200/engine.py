@@ -338,7 +338,8 @@ class Engine:
         self._check(self.lib.lh_snapshot_device(self.h, C.byref(v)))
         return v
 
-    def snapshot_reduce(self, percentiles) -> Reduced:
+    def _reduce_into(self, fn, percentiles) -> Reduced:
+        """fn(ctx, ps, np, counts, sums, avgs, pkeys, pvals): lh_snapshot_reduce or lh_window_reduce."""
         ps = np.ascontiguousarray(percentiles, dtype=np.float64)
         npct = ps.size
         H = self.H
@@ -347,10 +348,12 @@ class Engine:
         avgs = np.zeros(H, dtype=np.float64)
         pkeys = np.zeros((H, npct), dtype=np.int32)
         pvals = np.zeros((H, npct), dtype=np.float64)
-        self._check(self.lib.lh_snapshot_reduce(self.h, ps.ctypes.data if npct else 0, npct, counts.ctypes.data,
-                                                sums.ctypes.data, avgs.ctypes.data, pkeys.ctypes.data,
-                                                pvals.ctypes.data))
+        self._check(fn(self.h, ps.ctypes.data if npct else 0, npct, counts.ctypes.data, sums.ctypes.data,
+                       avgs.ctypes.data, pkeys.ctypes.data, pvals.ctypes.data))
         return Reduced(counts, sums, avgs, pkeys, pvals)
+
+    def snapshot_reduce(self, percentiles) -> Reduced:
+        return self._reduce_into(self.lib.lh_snapshot_reduce, percentiles)
 
     def snapshot_reduce_async(self, percentiles) -> tuple:
         """Enqueue the reduction; returns an opaque handle for snapshot_result()."""
@@ -371,15 +374,19 @@ class Engine:
                                                 pkeys.ctypes.data, pvals.ctypes.data))
         return Reduced(counts, sums, avgs, pkeys, pvals)
 
-    def snapshot_export(self) -> Sparse:
+    def _export_from(self, fn) -> Sparse:
+        """fn(ctx, lh_sparse *): lh_snapshot_export or lh_window_export; the lists are copied out of the library's buffers."""
         sp = L.lh_sparse()
-        self._check(self.lib.lh_snapshot_export(self.h, C.byref(sp)))
+        self._check(fn(self.h, C.byref(sp)))
         total = int(sp.total_entries)
         offsets = np.ctypeslib.as_array(sp.offsets, shape=(self.H + 1,)).copy()
         keys = np.ctypeslib.as_array(sp.keys, shape=(total,)).copy() if total else np.zeros(0, np.int16)
         counts = np.ctypeslib.as_array(sp.counts, shape=(total,)).copy() if total else np.zeros(0, np.uint64)
         deltas = np.ctypeslib.as_array(sp.counter_deltas, shape=(self.C,)).copy()
         return Sparse(offsets, keys, counts, deltas)
+
+    def snapshot_export(self) -> Sparse:
+        return self._export_from(self.lib.lh_snapshot_export)
 
     def snapshot_copy_histogram(self, histogram_id: int) -> np.ndarray:
         out = np.zeros(65536, dtype=np.uint64)
@@ -398,6 +405,28 @@ class Engine:
         finally:
             self.snapshot_end()
         return red, sp
+
+    # ---- windows: sums over the last K folded snapshots (K = 0: every snapshot since configure), on the device
+    def window_configure(self, intervals: int):
+        self._check(self.lib.lh_window_configure(self.h, intervals))
+
+    def window_release(self):
+        self._check(self.lib.lh_window_release(self.h))
+
+    def window_fold(self):
+        """Fold the open snapshot (after any all-reduce) into the window; once per snapshot."""
+        self._check(self.lib.lh_window_fold(self.h))
+
+    def window_reduce(self, percentiles) -> Reduced:
+        return self._reduce_into(self.lib.lh_window_reduce, percentiles)
+
+    def window_export(self) -> Sparse:
+        return self._export_from(self.lib.lh_window_export)
+
+    def window_info(self) -> dict:
+        st = L.lh_window_stats()
+        self._check(self.lib.lh_window_info(self.h, C.byref(st)))
+        return {f: int(getattr(st, f)) for f, _ in L.lh_window_stats._fields_}
 
     # ---- probes / streams
     def compress(self, values: np.ndarray, mode: int = 0) -> np.ndarray:
